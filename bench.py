@@ -4,6 +4,7 @@ per-request hot path, N replicas on N GPUs of one node (no collective: requests 
 
   python bench.py --gpus N --steps K --warmup W            # this repo's sm_100a path
   python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the oracle port of the reference path
+  python bench.py ... --dump-outputs DIR                   # + DIR/prob.npy: what the last timed step computed
 
 A "step" is one pass of the hot path over one batch of 8 synthetic 3x224x224 images.
   value : whole-job inferences/s with inputs already resident in HBM (4 ExecutionContexts on 4 streams,
@@ -184,6 +185,14 @@ def run_reference(args):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out_dir: str, arrays: dict):
+    """The arrays the headline leg's last timed step returned (ResNet-50 `prob`, [8, 1000]: 32 KB), one float32
+    DIR/<binding>.npy each, so that two builds can be compared output for output on identical seeded inputs."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.asarray(a, np.float32))
+
+
 def run_config2(capi, builder, peaks_int8_tops: float = 4500.0):
     """BASELINE.json configs[2]: ResNet-152 INT8, batch 32, dynamic batching (examples/03_Batching), 8 streams, 1 GPU.
     Device-resident throughput of 8 execution contexts + the end-to-end rate of single-image requests merged by
@@ -271,9 +280,12 @@ def run_b200(args):
     sampler = ClockSampler(local)
     barrier()
     sampler.start()
-    elapsed_ms, launches_per_step = capi.device_throughput(blob, CONTEXTS, BATCH, args.steps, max(args.warmup, 3), ring)
+    elapsed_ms, launches_per_step, *last = capi.device_throughput(blob, CONTEXTS, BATCH, args.steps, max(args.warmup, 3), ring,
+                                                                  return_outputs=args.dump_outputs is not None)
     barrier()
     clocks = sampler.stop()
+    if last and rank == 0:
+        dump_outputs(args.dump_outputs, last[0])
     elapsed_ms = max_over_ranks(elapsed_ms)
     ms_per_step = elapsed_ms / args.steps
     value = world * args.steps * BATCH / (elapsed_ms * 1e-3)
@@ -459,7 +471,11 @@ def main():
     ap.add_argument("--cpu-batches", type=int, default=20)
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--no-config2", action="store_true", help="skip the secondary ResNet-152 INT8 line (BASELINE configs[2])")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the headline leg's last timed step (its input: "
+                    f"batch (steps - 1) mod {RING} of the seeded input ring) as DIR/<binding>.npy, float32")
     args = ap.parse_args()
+    if args.dump_outputs is not None and args.impl == "reference":
+        ap.error("--dump-outputs applies to the b200 implementation")
     if args.gpus > 1 and "WORLD_SIZE" not in os.environ:
         # convenience: re-launch ourselves one rank per GPU (the driver does this itself via torchrun)
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", f"--nproc-per-node={args.gpus}",

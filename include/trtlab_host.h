@@ -66,9 +66,13 @@ int trt_workspace_infer(const void* blob, size_t nbytes, const void* input, size
  * requests cut from a 3-segment ring (which therefore wraps); output and device time of the last request */
 int trt_cyclic_infer(const void* blob, size_t nbytes, int batch, const void* input, size_t input_bytes, void* output,
                      size_t output_bytes, int managed_runtime, int rounds, double* compute_seconds);
-/* device-resident throughput of `contexts` concurrent execution contexts (inputs cycled through a device ring) */
+/* device-resident throughput of `contexts` concurrent execution contexts (inputs cycled through a device ring).
+ * Timed step i runs on context i % contexts with input ring[i % ring_batches].  last_outputs (may be NULL): after the
+ * timed region, the `batch` rows of every output binding computed by the last timed step, back to back in binding
+ * order; last_outputs_bytes must equal their total size */
 int trt_device_throughput(const void* blob, size_t nbytes, int contexts, int batch, int steps, int warmup,
-                          const void* host_ring, int ring_batches, double* elapsed_ms, int* launches_per_step);
+                          const void* host_ring, int ring_batches, double* elapsed_ms, int* launches_per_step,
+                          void* last_outputs, size_t last_outputs_bytes);
 
 #ifdef __cplusplus
 }

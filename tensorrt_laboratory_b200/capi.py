@@ -101,7 +101,7 @@ SYMBOLS = [
     ("trt_manager_bench_window", _I, [_VP, _S, _I, _SZ, _SZ, _SZ, C.POINTER(_D), C.POINTER(_D), _SZ, C.POINTER(_SZ)]),
     ("trt_manager_bench_windows", _I, [_VP, _S, _I, _SZ, _SZ, _SZ, _SZ, C.POINTER(_D), C.POINTER(_D), _SZ, C.POINTER(_SZ)]),
     ("trt_timed_pipeline", _I, [_VP, _SZ, _I, C.POINTER(C.c_float), C.POINTER(C.c_float), C.POINTER(C.c_float)]),
-    ("trt_device_throughput", _I, [_VP, _SZ, _I, _I, _I, _I, _VP, _I, C.POINTER(_D), C.POINTER(_I)]),
+    ("trt_device_throughput", _I, [_VP, _SZ, _I, _I, _I, _I, _VP, _I, C.POINTER(_D), C.POINTER(_I), _VP, _SZ]),
     ("trt_workspace_infer", _I, [_VP, _SZ, _VP, _SZ, _VP, _SZ, _I, _I]),
     ("trt_cyclic_infer", _I, [_VP, _SZ, _I, _VP, _SZ, _VP, _SZ, _I, _I, C.POINTER(_D)]),
 ]
@@ -588,14 +588,31 @@ def timed_pipeline(blob: bytes, iters: int = 20):
     return dict(h2d_ms=a.value, compute_ms=b.value, d2h_ms=c.value)
 
 
-def device_throughput(blob: bytes, contexts: int, batch: int, steps: int, warmup: int, ring: np.ndarray):
-    """-> (elapsed_ms, kernel launches per step).  ``ring``: [R, batch, C, H, W] host array (cast to the input dtype)."""
+def device_throughput(blob: bytes, contexts: int, batch: int, steps: int, warmup: int, ring: np.ndarray,
+                      return_outputs: bool = False):
+    """-> (elapsed_ms, kernel launches per step), and with ``return_outputs`` a third item: {output binding name:
+    [batch, ...] array} computed by the last timed step (input ``ring[(steps - 1) % R]``).  ``ring``: [R, batch, C, H, W]
+    host array (cast to the input dtype)."""
     ring = np.ascontiguousarray(ring, dtype=input_np_dtype(blob))
+    outs = []
+    if return_outputs:
+        meta = Engine(blob, inspect_only=True)
+        outs = [b for b in meta.bindings if not b["is_input"]]
+        meta.destroy()
+    flat = np.empty(sum(batch * b["item_bytes"] for b in outs), np.uint8)  # the C side writes them back to back
     ms = _D()
     nl = _I()
     check(load().trt_device_throughput(blob, len(blob), contexts, batch, steps, warmup, ring.ctypes.data,
-                                       ring.shape[0], C.byref(ms), C.byref(nl)))
-    return ms.value, nl.value
+                                       ring.shape[0], C.byref(ms), C.byref(nl),
+                                       flat.ctypes.data if return_outputs else None, flat.nbytes))
+    if not return_outputs:
+        return ms.value, nl.value
+    arrays, off = {}, 0
+    for b in outs:
+        n = batch * b["item_bytes"]
+        arrays[b["name"]] = flat[off:off + n].copy().view(b["np_dtype"]).reshape((batch,) + b["shape"])
+        off += n
+    return ms.value, nl.value, arrays
 
 
 def _single_io(blob: bytes):

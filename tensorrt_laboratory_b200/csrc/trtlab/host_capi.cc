@@ -365,7 +365,8 @@ int trt_cyclic_infer(const void* blob, size_t nbytes, int batch, const void* inp
 }
 
 int trt_device_throughput(const void* blob, size_t nbytes, int contexts, int batch, int steps, int warmup,
-                          const void* host_ring, int ring_batches, double* elapsed_ms, int* launches_per_step) {
+                          const void* host_ring, int ring_batches, double* elapsed_ms, int* launches_per_step,
+                          void* last_outputs, size_t last_outputs_bytes) {
     if (!blob || contexts < 1 || steps < 1 || !host_ring || ring_batches < 1 || !elapsed_ms) return fail(B2_EINVAL, "bad arguments");
     b2_runtime* rt = nullptr;
     b2_engine* eng = nullptr;
@@ -396,6 +397,17 @@ int trt_device_throughput(const void* blob, size_t nbytes, int contexts, int bat
         for (int d = 0; d < nd; ++d) n *= size_t(dims[d]);
         bytes[i] = n * size_t(b2_engine_max_batch(eng));
         if (b2_engine_binding_is_input(eng, i)) in_id = i;
+    }
+    auto batch_bytes = [&](int i) { return bytes[size_t(i)] / size_t(b2_engine_max_batch(eng)) * size_t(batch); };
+    if (last_outputs) {
+        size_t want = 0;
+        for (int i = 0; i < nb; ++i)
+            if (i != in_id) want += batch_bytes(i);
+        if (last_outputs_bytes != want) {
+            b2_engine_destroy(eng);
+            b2_runtime_destroy(rt);
+            return fail(B2_EINVAL, "last_outputs_bytes %zu != %zu (the output bindings of one batch)", last_outputs_bytes, want);
+        }
     }
     struct Ctx {
         b2_context* c = nullptr;
@@ -501,6 +513,15 @@ int trt_device_throughput(const void* blob, size_t nbytes, int contexts, int bat
         float ms = 0.f;
         if (status == B2_OK && cuda_ok(cudaEventElapsedTime(&ms, start, stop), "elapsed")) *elapsed_ms = ms;
         if (launches_per_step) *launches_per_step = b2_context_nb_launches(ctx[0].c, batch);
+        if (status == B2_OK && last_outputs) {  // outside the timed region; no later step used this context
+            const Ctx& x = ctx[size_t((steps - 1) % contexts)];
+            char* dst = static_cast<char*>(last_outputs);
+            for (int i = 0; i < nb; ++i) {
+                if (i == in_id) continue;
+                if (!cuda_ok(cudaMemcpy(dst, x.bind[size_t(i)], batch_bytes(i), cudaMemcpyDeviceToHost), "last outputs download")) break;
+                dst += batch_bytes(i);
+            }
+        }
     }
     bg_stop = true;
     if (bg.joinable()) bg.join();

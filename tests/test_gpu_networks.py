@@ -215,6 +215,17 @@ def test_device_throughput_harness(rn50_session):
     assert ms > 0 and launches == 56
 
 
+def test_device_throughput_returns_the_last_steps_outputs(rn50_session):
+    """What `bench.py --dump-outputs` writes: step 7 of 8 ran on context 1 with input ring[7 % 3]."""
+    ring = weights.synthetic_input(8, seed=7, ring=3)
+    ms, _, outs = capi.device_throughput(rn50_session["blob"], contexts=2, batch=8, steps=8, warmup=4, ring=ring,
+                                         return_outputs=True)
+    assert ms > 0 and list(outs) == ["prob"] and outs["prob"].shape == (8, 1000) and outs["prob"].dtype == np.float32
+    want = rn50_session["sess"].infer(ring[1])["prob"]
+    assert (outs["prob"].argmax(1) == want.argmax(1)).all()
+    assert (np.abs(outs["prob"] - want) / want.max(1, keepdims=True)).max() <= 1e-4
+
+
 def test_enqueue_argument_validation(rn50_session):
     import ctypes as C
     lib = capi.load()

@@ -1,19 +1,17 @@
 """CPU: model front-ends (prototxt parser, generated ResNets, ONNX-lite) and the lowering pass."""
+import gzip
 import os
 
 import numpy as np
 import pytest
 
 from tensorrt_laboratory_b200 import graph, onnx_lite, weights
-
-REF = "/root/reference"
-needs_ref = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "models")), reason="reference tree not mounted")
+from tests.helpers import GOLDEN
 
 
-@needs_ref
 @pytest.mark.parametrize("depth,nlayers", [(50, 228), (152, 670)])
 def test_generated_resnet_equals_reference_prototxt(depth, nlayers):
-    with open(os.path.join(REF, f"models/ResNet-{depth}-deploy.prototxt")) as f:
+    with gzip.open(os.path.join(GOLDEN, f"ResNet-{depth}-deploy.prototxt.gz"), "rt") as f:
         parsed = graph.parse_prototxt(f.read())
     gen = graph.resnet_caffe(depth)
     assert parsed["input_dims"] == gen["input_dims"] == [1, 3, 224, 224]
@@ -80,14 +78,13 @@ def test_weights_are_deterministic_and_specified():
     assert x.shape == (3, 2, 3, 224, 224) and x.dtype == np.float32
 
 
-@needs_ref
 def test_onnx_lite_reads_reference_mnist():
-    model = onnx_lite.load_model(os.path.join(REF, "models/onnx/mnist-v1.3/model.onnx"))
+    model = onnx_lite.load_model(os.path.join(GOLDEN, "mnist_v1_3_model.onnx"))
     assert [n["op"] for n in model["nodes"]] == ["Reshape", "Conv", "Add", "Relu", "MaxPool", "Conv", "Add", "Relu",
                                                  "MaxPool", "Reshape", "MatMul", "Add"]
     net, w = onnx_lite.mnist_to_caffe_like(model)
     assert graph.infer_shapes(net)[net["layers"][-1]["tops"][0]] == (10, 1, 1)
-    x = onnx_lite.load_tensor(os.path.join(REF, "models/onnx/mnist-v1.3/test_data_set_0/input_0.pb"))
+    x = onnx_lite.load_tensor(os.path.join(GOLDEN, "mnist_v1_3_input_0.pb"))
     assert x.shape == (1, 1, 28, 28)
     # the committed fixture is exactly what the decoder produces
     from tests import helpers

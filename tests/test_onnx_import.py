@@ -8,7 +8,7 @@ from oracle.caffe_forward import caffe_forward
 from tensorrt_laboratory_b200 import builder, graph, onnx_import, onnx_lite, weights
 from tests import helpers
 
-MNIST_ONNX = "/root/reference/models/onnx/mnist-v1.3/model.onnx"
+MNIST_ONNX = os.path.join(helpers.GOLDEN, "mnist_v1_3_model.onnx")
 
 
 def _same_lowering(a, b, tol=1e-6):
@@ -47,7 +47,6 @@ def test_round_trip_preserves_the_forward_pass():
     np.testing.assert_allclose(caffe_forward(net2, w2, x), caffe_forward(net, w, x), rtol=1e-5, atol=1e-6)
 
 
-@pytest.mark.skipif(not os.path.exists(MNIST_ONNX), reason="the reference tree is only mounted in the build container")
 def test_reference_mnist_model_through_the_generic_importer():
     model = onnx_lite.load_model(MNIST_ONNX)
     net, w = onnx_import.import_onnx(model, name="mnist-v1.3")     # Conv(SAME_UPPER)+Add, Relu, MaxPool, Reshape, MatMul+Add
