@@ -45,6 +45,9 @@ class Bindings;
 class Runtime;
 class InferenceManager;
 
+// bytes of one element of a B2_DT_* binding dtype (the one place binding sizes are derived from)
+size_t dtype_size(int dtype);
+
 // ------------------------------------------------------------------------------------------------
 // memory tags used by FixedBuffers<Host, Device> (reference trtlab/cuda memory types:
 // trtlab/cuda/include/trtlab/cuda/memory/device_memory.h:36-84)

@@ -24,7 +24,70 @@ _HEADER = struct.Struct("<8sIIIIIIQQ64s16x")
 _TENSOR = struct.Struct("<64sIIIIIif4x")  # ... binding, scale (INT8 tensors: real value = q * scale; 0 = fp16 / fp32 tensor)
 _OP = struct.Struct("<64sIiiiiIIIIIIIIIIIQQQQIIII")
 _BINDING = struct.Struct("<64sIIiI8i16x")
-assert _HEADER.size == 128 and _TENSOR.size == 96 and _OP.size == 176 and _BINDING.size == 128
+_INPUT_NORM = struct.Struct("<4f4fII4B4x")  # mean[4], inv_std[4], crop_top, crop_left, perm[4]
+assert _HEADER.size == 128 and _TENSOR.size == 96 and _OP.size == 176 and _BINDING.size == 128 and _INPUT_NORM.size == 48
+DT_FLOAT, DT_HALF, DT_UINT8 = 0, 1, 5  # B2_DT_* of include/b200infer.h (5 = TensorRT's kUINT8)
+
+# torchvision's ImageNet normalisation in pixel units (0..255): ToTensor's /255 folded into mean and std
+TORCHVISION_MEAN = tuple(255.0 * v for v in (0.485, 0.456, 0.406))
+TORCHVISION_STD = tuple(255.0 * v for v in (0.229, 0.224, 0.225))
+
+
+def center_crop_offsets(src_hw: Sequence[int], hw: Sequence[int]):
+    """(top, left) of an H x W crop centred in a src_h x src_w image, rounded like torchvision's CenterCrop."""
+    return int(round((src_hw[0] - hw[0]) / 2.0)), int(round((src_hw[1] - hw[1]) / 2.0))
+
+
+def image_norm(image: Optional[dict], chw: Sequence[int]) -> dict:
+    """Validated normalisation of a uint8 image binding feeding a [C, H, W] input:
+    ``image`` = dict(mean=..., std=..., reverse_channels=False, src_hw=None) in pixel units (a scalar or C values each;
+    defaults mean 0, std 1, src_hw = (H, W)).  -> dict(mean, inv_std: float32 [C], perm, src_hw, top, left)."""
+    c, h, w = (int(v) for v in chw)
+    image = dict(image or {})
+    unknown = set(image) - {"mean", "std", "reverse_channels", "src_hw"}
+    if unknown:
+        raise ValueError(f"image: unknown keys {sorted(unknown)}")
+    if not 1 <= c <= 4:
+        raise ValueError(f"uint8 image inputs carry 1..4 channels, this network takes {c}")
+
+    def per_channel(key, dflt):
+        v = np.asarray(image.get(key, dflt), dtype=np.float64).reshape(-1)
+        if v.size == 1:
+            v = np.repeat(v, c)
+        if v.size != c or not np.all(np.isfinite(v)):
+            raise ValueError(f"image: {key} needs 1 or {c} finite values, got {image.get(key)!r}")
+        return v
+
+    mean, std = per_channel("mean", 0.0), per_channel("std", 1.0)
+    if np.any(std == 0):
+        raise ValueError("image: std must be non-zero")
+    inv_std = (1.0 / std).astype(np.float32)  # computed in float64, rounded once
+    if not np.all(np.isfinite(inv_std)) or np.any(inv_std == 0):
+        raise ValueError("image: 1/std is not a finite non-zero float32")
+    reverse = bool(image.get("reverse_channels", False))
+    if reverse and c != 3:
+        raise ValueError("image: reverse_channels (RGB <-> BGR) needs 3 channels")
+    src_hw = tuple(int(v) for v in (image.get("src_hw") or (h, w)))
+    if len(src_hw) != 2 or src_hw[0] < h or src_hw[1] < w:
+        raise ValueError(f"image: a {h}x{w} crop does not fit a source of {src_hw}")
+    top, left = center_crop_offsets(src_hw, (h, w))
+    return dict(mean=mean.astype(np.float32), inv_std=inv_std, perm=tuple(range(c))[::-1] if reverse else tuple(range(c)),
+                src_hw=src_hw, top=top, left=left, chw=(c, h, w))
+
+
+def preprocess_u8(x: np.ndarray, chw: Sequence[int], image: Optional[dict] = None) -> np.ndarray:
+    """The semantics of a uint8 image binding, in numpy: uint8 [N, src_h, src_w, C] -> float32 [N, C, H, W], what the
+    fp32 binding of the same engine receives.  Centre crop, channel order ``perm``, then per channel
+    ``(float32(x) - mean) * inv_std`` in float32 (one subtract, one multiply); the engine's first kernel computes these exact
+    values before rounding them to fp16."""
+    nrm = image_norm(image, chw)
+    c, h, w = nrm["chw"]
+    x = np.asarray(x)
+    if x.dtype != np.uint8 or x.ndim != 4 or x.shape[1:] != nrm["src_hw"] + (c,):
+        raise ValueError(f"expected uint8 [N, {nrm['src_hw'][0]}, {nrm['src_hw'][1]}, {c}], got {x.dtype} {x.shape}")
+    crop = x[:, nrm["top"]:nrm["top"] + h, nrm["left"]:nrm["left"] + w, :][..., list(nrm["perm"])].astype(np.float32)
+    y = (crop - nrm["mean"]) * nrm["inv_std"]
+    return np.ascontiguousarray(y.transpose(0, 3, 1, 2))
 
 
 def _roundup(v: int, m: int) -> int:
@@ -103,11 +166,14 @@ def _name(s: str) -> bytes:
 
 def build_plan(lowered: dict, precision: int = PREC_FP16, max_batch: int = 8,
                outputs: Optional[Sequence[str]] = None, name: Optional[str] = None, stem_s2d: bool = True,
-               pack_weights: bool = True, input_dtype: str = "f32") -> bytes:
+               pack_weights: bool = True, input_dtype: str = "f32", image: Optional[dict] = None) -> bytes:
     """Serialize ``lowered`` (from :func:`graph.lower` with weights) into a plan blob.
 
     ``input_dtype``: "f32" = the reference's binding contract (pybind casts inputs to float, infer.cc:435-441);
-    "f16" (fp16 engines only) = the secondary mode of SURVEY.md §8(d): half the H2D bytes per request.
+    "f16" (fp16 engines only) = the secondary mode of SURVEY.md §8(d): half the H2D bytes per request;
+    "u8" (fp16 and INT8 engines, 1..4 channels) = decoded images, uint8 [src_h, src_w, C] per item, a quarter of the fp32
+    bytes: the input cast crops, orders and normalises them as :func:`preprocess_u8` with ``image`` (see
+    :func:`image_norm`) specifies.
 
     ``outputs``: tensor names to expose as output bindings (default: the graph output).  4-D activation
     outputs get an ``OUTPUT_CAST`` to fp32 NCHW; vector outputs (fc / softmax) are written in place.
@@ -159,10 +225,16 @@ def build_plan(lowered: dict, precision: int = PREC_FP16, max_batch: int = 8,
     # input binding + cast
     cin, hin, win = lowered["input_shape"]
     t_in = add_tensor(lowered["input"])
-    if input_dtype not in ("f32", "f16") or (input_dtype == "f16" and precision_fp != PREC_FP16):
-        raise ValueError("input_dtype is 'f32' (the reference's binding contract) or, for fp16 engines, 'f16'")
-    bindings.append(dict(name=lowered["input"], is_input=1, dtype=1 if input_dtype == "f16" else 0, tensor=t_in,
-                         dims=[cin, hin, win]))
+    if input_dtype not in ("f32", "f16", "u8") or (input_dtype != "f32" and precision_fp != PREC_FP16):
+        raise ValueError("input_dtype is 'f32' (the reference's binding contract) or, for fp16 / INT8 engines, 'f16' or 'u8'")
+    if image is not None and input_dtype != "u8":
+        raise ValueError("image= describes a uint8 input binding: pass input_dtype='u8'")
+    norm = image_norm(image, (cin, hin, win)) if input_dtype == "u8" else None
+    if norm is not None:
+        bindings.append(dict(name=lowered["input"], is_input=1, dtype=DT_UINT8, tensor=t_in, dims=[*norm["src_hw"], cin]))
+    else:
+        bindings.append(dict(name=lowered["input"], is_input=1, dtype=DT_HALF if input_dtype == "f16" else DT_FLOAT, tensor=t_in,
+                             dims=[cin, hin, win]))
     ops.append(dict(name="cast:" + lowered["input"], type=OP_INPUT_CAST, inp=-1, res=-1, out=t_in, binding=0))
     # fp16 stem: a stride-2 conv that is the only reader of a thin (<= 4 channel) even-width input runs on a
     # horizontally space-to-depth packed copy of the input (see stem_s2d_transform)
@@ -265,6 +337,14 @@ def build_plan(lowered: dict, precision: int = PREC_FP16, max_batch: int = 8,
             bindings.append(dict(name=oname, is_input=0, dtype=0, tensor=ti, dims=[trec["c"], trec["h"], trec["w"]]))
             ops.append(dict(name="cast:" + oname, type=OP_OUTPUT_CAST, inp=ti, res=-1, out=-1, binding=bidx))
 
+    if norm is not None:  # behind every weight, so the weight offsets are those of the fp32-binding plan
+        while len(payload) % 16:
+            payload.append(0)
+        perm = list(norm["perm"]) + [0] * (4 - cin)
+        ops[0].update(b_off=len(payload), b_bytes=_INPUT_NORM.size)
+        payload.extend(_INPUT_NORM.pack(*np.pad(norm["mean"], (0, 4 - cin)).tolist(), *np.pad(norm["inv_std"], (0, 4 - cin)).tolist(),
+                                        norm["top"], norm["left"], *perm))
+
     tables = _HEADER.size + len(tensors) * _TENSOR.size + len(ops) * _OP.size + len(bindings) * _BINDING.size
     payload_offset = _roundup(tables, 256)
     blob = bytearray()
@@ -287,17 +367,31 @@ def build_plan(lowered: dict, precision: int = PREC_FP16, max_batch: int = 8,
     return bytes(blob)
 
 
-def build_resnet_plan(depth: int = 50, precision: int = PREC_FP16, max_batch: int = 8, seed: int = 0,
-                      input_dtype: str = "f32", calib_batch: int = 8) -> bytes:
-    """Convenience: generated Caffe-v1 ResNet + deterministic weights -> plan.  PREC_INT8: post-training quantization
-    calibrated (max-abs) on ``calib_batch`` synthetic images (seed 4321), see quantize.py."""
+def resnet_lowered(depth: int = 50, precision: int = PREC_FP16, seed: int = 0, calib_batch: int = 8,
+                   image: Optional[dict] = None) -> dict:
+    """Generated Caffe-v1 ResNet + deterministic weights, lowered.  PREC_INT8: quantized, calibrated (max-abs) on
+    ``calib_batch`` synthetic inputs (seed 4321) -- with ``image``, on :func:`preprocess_u8` of synthetic uint8 images, the
+    values a uint8 binding feeds the network."""
     from . import weights as Wt
     net = G.resnet_caffe(depth)
     low = G.lower(net, Wt.random_weights(net, seed))
     if precision == PREC_INT8:
         from . import quantize
-        low = quantize.quantize_lowered(low, Wt.synthetic_input(calib_batch, seed=4321))
-    return build_plan(low, precision, max_batch, input_dtype=input_dtype)
+        if image is None:
+            calib = Wt.synthetic_input(calib_batch, seed=4321)
+        else:
+            chw = low["input_shape"]
+            src_hw = image_norm(image, chw)["src_hw"]
+            calib = preprocess_u8(Wt.synthetic_image_u8(calib_batch, src_hw, chw[0], seed=4321), chw, image)
+        low = quantize.quantize_lowered(low, calib)
+    return low
+
+
+def build_resnet_plan(depth: int = 50, precision: int = PREC_FP16, max_batch: int = 8, seed: int = 0,
+                      input_dtype: str = "f32", calib_batch: int = 8, image: Optional[dict] = None) -> bytes:
+    """Convenience: :func:`resnet_lowered` -> plan (``input_dtype`` / ``image`` as in :func:`build_plan`)."""
+    low = resnet_lowered(depth, precision, seed, calib_batch, image if input_dtype == "u8" else None)
+    return build_plan(low, precision, max_batch, input_dtype=input_dtype, image=image)
 
 
 def single_conv_net(cin: int, h: int, w: int, cout: int, k: int, stride: int, pad: int, relu: bool = True,

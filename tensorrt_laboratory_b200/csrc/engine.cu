@@ -12,6 +12,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 #include <map>
 #include <memory>
 #include <mutex>
@@ -126,6 +127,7 @@ struct Binding {
     int nd;
     int32_t dims[8];
     size_t item_bytes;
+    b2k::U8Norm norm{};  // B2_DT_UINT8 input: source geometry, crop and normalisation (from the plan's InputNormRec)
 };
 
 enum LKind { L_INPUT_CAST, L_CONV_TC, L_CONV_SIMT, L_MAXPOOL, L_AVGPOOL, L_FC, L_SOFTMAX, L_OUTPUT_CAST, L_NET, L_TAIL, L_QUANTIZE, L_CONV_I8, L_AVGPOOL_I8, L_OUTPUT_CAST_I8 };
@@ -153,7 +155,8 @@ struct Launch {
     const void* w = nullptr;
     const float* bias = nullptr;
     int in_binding = -1, out_binding = -1;
-    bool src_half = false;  // input cast: the binding is fp16
+    int src_dtype = B2_DT_FLOAT;  // input cast: dtype of the binding (fp32, fp16 or uint8 HWC)
+    b2k::U8Norm norm{};           // input cast of a uint8 binding: passed to the kernel by value
     int max_blocks = 0;     // input cast: grid cap (option input_ctas), 0 = one thread per element group
     int side_join = -1;     // see Op::side_join (launch index == op index)
     std::shared_ptr<NetRun> net;  // L_NET
@@ -439,15 +442,19 @@ int parse_blob(const void* blob, size_t nbytes, b2_engine* e, const uint8_t** pa
         b.tensor = r.tensor;
         b.nd = r.nd;
         if (r.nd == 0 || r.nd > 8) return fail(B2_EINVAL, "plan: binding %s has bad rank", b.name.c_str());
-        // fp32 is the reference's binding contract; fp16 INPUT bindings are the secondary mode of fp16 engines
-        if (r.dtype != B2_DT_FLOAT && !(r.dtype == B2_DT_HALF && b.is_input && h.precision == B2_PREC_FP16))
-            return fail(B2_EINVAL, "plan: binding %s: bindings are fp32 (inputs of fp16 engines may be fp16)", b.name.c_str());
+        // fp32 is the reference's binding contract; fp16 INPUT bindings are the secondary mode of fp16 engines, uint8 HWC
+        // image inputs that of fp16 and INT8 engines (both have the fp16 stem)
+        if (r.dtype != B2_DT_FLOAT && !(r.dtype == B2_DT_HALF && b.is_input && h.precision == B2_PREC_FP16) &&
+            !(r.dtype == B2_DT_UINT8 && b.is_input && h.precision != B2_PREC_FP32))
+            return fail(B2_EINVAL, "plan: binding %s: bindings are fp32 (inputs of fp16 engines may be fp16, of fp16 / INT8 "
+                                   "engines uint8)", b.name.c_str());
+        if (r.dtype == B2_DT_UINT8 && r.nd != 3) return fail(B2_EINVAL, "plan: uint8 binding %s is not {H, W, C}", b.name.c_str());
         size_t n = 1;
         for (uint32_t d = 0; d < 8; ++d) {
             b.dims[d] = d < r.nd ? r.dims[d] : 0;
             if (d < r.nd) n *= size_t(r.dims[d]);
         }
-        b.item_bytes = n * (r.dtype == B2_DT_HALF ? 2 : 4);
+        b.item_bytes = n * (r.dtype == B2_DT_UINT8 ? 1 : r.dtype == B2_DT_HALF ? 2 : 4);
         e->bindings.push_back(b);
     }
     // cast ops move a binding <-> a tensor: the caller sizes its Buffers from the BINDING dims, so the two must agree
@@ -459,8 +466,46 @@ int parse_blob(const void* blob, size_t nbytes, b2_engine* e, const uint8_t** pa
         size_t n = 1;
         for (int d = 0; d < b.nd; ++d) n *= size_t(b.dims[d] > 0 ? b.dims[d] : 0);
         const bool s2d = r.type == OP_INPUT_CAST && r.k == 2;  // (its geometry is re-checked when the launch plan is built)
-        if (b.is_input != (r.type == OP_INPUT_CAST) || (!s2d && n != size_t(t.c) * t.h * t.w))
+        const bool u8 = b.dtype == B2_DT_UINT8;
+        if (b.is_input != (r.type == OP_INPUT_CAST) || (!s2d && !u8 && n != size_t(t.c) * t.h * t.w))
             return fail(B2_EINVAL, "plan: cast op %s: binding %s and tensor %s disagree", op.name.c_str(), b.name.c_str(), t.name.c_str());
+        if (r.type != OP_INPUT_CAST) continue;
+        if (r.b_bytes != (u8 ? sizeof(InputNormRec) : 0))
+            return fail(B2_EINVAL, "plan: input cast %s: %llu normalisation bytes for a %s binding", op.name.c_str(),
+                        (unsigned long long)r.b_bytes, u8 ? "uint8" : "non-uint8");
+        if (!u8) continue;
+        // uint8 HWC image: {src_h, src_w, C} -> the tensor's H x W crop (s2d: the tensor holds W/2 + pad_l + pad_r pairs)
+        InputNormRec nr;
+        memcpy(&nr, base + h.payload_offset + r.b_off, sizeof nr);  // (inside the payload: checked with the op)
+        const int64_t src_h = b.dims[0], src_w = b.dims[1], C = b.dims[2];
+        const int64_t H = t.h, W = s2d ? 2 * (int64_t(t.w) - int64_t(r.pad_) - int64_t(r.stride)) : int64_t(t.w);
+        if (src_h < 1 || src_w < 1 || C < 1 || C > 4 || (!s2d && int64_t(t.c) != C) || t.c_phys != 8 || W < 1)
+            return fail(B2_EINVAL, "plan: uint8 binding %s {%lld, %lld, %lld} does not fit tensor %s", b.name.c_str(),
+                        (long long)src_h, (long long)src_w, (long long)C, t.name.c_str());
+        if (int64_t(nr.crop_top) + H > src_h || int64_t(nr.crop_left) + W > src_w)
+            return fail(B2_EINVAL, "plan: uint8 binding %s: crop %lldx%lld at (%u, %u) outside the %lldx%lld source", b.name.c_str(),
+                        (long long)H, (long long)W, nr.crop_top, nr.crop_left, (long long)src_h, (long long)src_w);
+        unsigned seen = 0;
+        for (int c = 0; c < C; ++c) {
+            if (nr.perm[c] >= C || (seen & (1u << nr.perm[c])))
+                return fail(B2_EINVAL, "plan: uint8 binding %s: channel order is not a permutation of 0..%lld", b.name.c_str(),
+                            (long long)C - 1);
+            seen |= 1u << nr.perm[c];
+            if (!std::isfinite(nr.mean[c]) || !std::isfinite(nr.inv_std[c]) || nr.inv_std[c] == 0.f)
+                return fail(B2_EINVAL, "plan: uint8 binding %s: mean / inv_std of channel %d not finite or inv_std 0", b.name.c_str(), c);
+        }
+        for (int c = int(C); c < 4; ++c)  // entries past C are 0: the record agrees with the binding's channel count
+            if (nr.perm[c] != 0 || nr.mean[c] != 0.f || nr.inv_std[c] != 0.f)
+                return fail(B2_EINVAL, "plan: uint8 binding %s: normalisation entry %d set for a %lld-channel image", b.name.c_str(), c,
+                            (long long)C);
+        Binding& bm = e->bindings[size_t(r.binding)];
+        bm.norm.C = int(C), bm.norm.src_h = int(src_h), bm.norm.src_w = int(src_w);
+        bm.norm.top = int(nr.crop_top), bm.norm.left = int(nr.crop_left);
+        for (int c = 0; c < 4; ++c) {
+            bm.norm.mean[c] = c < C ? nr.mean[c] : 0.f;
+            bm.norm.inv_std[c] = c < C ? nr.inv_std[c] : 0.f;
+            bm.norm.perm[c] = c < C ? int(nr.perm[c]) : 0;
+        }
     }
     if (h.n_tactics) {  // tactic table written by an offline tuning run (b2_engine_get_tactics -> builder.attach_tactics)
         if (h.tactics_offset > nbytes || size_t(h.n_tactics) > (nbytes - h.tactics_offset) / sizeof(TacticRec))
@@ -1379,20 +1424,32 @@ int build_plan(b2_context* c, int batch, Plan** out) {
                 const Tensor& t = e->tensors[r.out];
                 L.kind = L_INPUT_CAST;
                 L.in_binding = r.binding;
-                L.src_half = e->bindings[r.binding].dtype == B2_DT_HALF;
+                const Binding& b = e->bindings[r.binding];
+                L.src_dtype = b.dtype;
                 L.out = tptr(r.out);
                 L.C = t.c, L.H = t.h, L.W = t.w, L.C_phys = t.c_phys;
-                L.k = int(r.k);  // 2: horizontal space-to-depth (tensor is [H, W/2, 8]; binding is [C, H, W])
+                L.k = int(r.k);  // 2: horizontal space-to-depth (tensor is [H, W/2, 8]; binding is [C, H, W] or [src_h, src_w, C])
                 L.max_blocks = c->input_ctas;
+                if (b.dtype == B2_DT_UINT8) {  // {src_h, src_w, C} cropped to the tensor's H x W (validated at load)
+                    L.norm = b.norm;
+                    L.C = b.norm.C;
+                    if (!half || t.c_phys != 8 || (r.k != 2 && int(t.c) != L.C))
+                        return fail(B2_EINVAL, "input cast %s: a uint8 binding needs the fp16 8-channel input layout", op.name.c_str());
+                }
                 if (r.k == 2) {  // pad_ / stride = zero pixels written left / right of every packed row
-                    const Binding& b = e->bindings[r.binding];
-                    if (!half || b.nd != 3 || b.dims[0] > 4 || t.c_phys != 8 || int(t.h) != b.dims[1] ||
-                        int(t.w) != b.dims[2] / 2 + int(r.pad_) + int(r.stride) || b.dims[2] % 2)
+                    const bool u8 = b.dtype == B2_DT_UINT8;
+                    const int C = u8 ? b.dims[2] : b.dims[0], H = u8 ? int(t.h) : b.dims[1];
+                    const int W = u8 ? 2 * (int(t.w) - int(r.pad_) - int(r.stride)) : b.dims[2];
+                    if (!half || b.nd != 3 || C > 4 || t.c_phys != 8 || int(t.h) != H || W < 2 ||
+                        int(t.w) != W / 2 + int(r.pad_) + int(r.stride) || W % 2)
                         return fail(B2_EINVAL, "input cast %s: inconsistent space-to-depth geometry", op.name.c_str());
-                    L.C = b.dims[0], L.W = b.dims[2];
+                    L.C = C, L.W = W;
                     L.pad = int(r.pad_), L.stride = int(r.stride);
                 }
-                L.bytes = double(batch) * t.h * t.w * (t.c * 4.0 + t.c_phys * elt);
+                if (b.dtype == B2_DT_UINT8)  // the crop's bytes in, the padded fp16 tensor out
+                    L.bytes = double(batch) * (double(L.H) * L.W * L.C + double(t.h) * t.w * t.c_phys * elt);
+                else
+                    L.bytes = double(batch) * t.h * t.w * (t.c * 4.0 + t.c_phys * elt);
                 break;
             }
             case b2plan::OP_QUANTIZE: {
@@ -1592,8 +1649,13 @@ int run_launch(const b2_engine* e, const Launch& L, void* const* bindings, cudaS
     void* out = L.out_binding >= 0 ? bindings[L.out_binding] : L.out;
     switch (L.kind) {
         case L_INPUT_CAST:
-            if (L.k == 2) return b2k::launch_input_cast_s2d(in, L.src_half, out, L.N, L.C, L.H, L.W, L.pad, L.stride, L.max_blocks, s);
-            return b2k::launch_input_cast(in, L.src_half, out, L.N, L.C, L.H, L.W, L.C_phys, half, L.max_blocks, s);
+            if (L.src_dtype == B2_DT_UINT8) {
+                if (L.k == 2) return b2k::launch_input_cast_u8_s2d(in, out, L.N, L.H, L.W, L.pad, L.stride, L.norm, L.max_blocks, s);
+                return b2k::launch_input_cast_u8_c8(in, out, L.N, L.H, L.W, L.norm, L.max_blocks, s);
+            }
+            if (L.k == 2)
+                return b2k::launch_input_cast_s2d(in, L.src_dtype == B2_DT_HALF, out, L.N, L.C, L.H, L.W, L.pad, L.stride, L.max_blocks, s);
+            return b2k::launch_input_cast(in, L.src_dtype == B2_DT_HALF, out, L.N, L.C, L.H, L.W, L.C_phys, half, L.max_blocks, s);
         case L_OUTPUT_CAST:
             return b2k::launch_output_cast(in, static_cast<float*>(out), L.N, L.C, L.H, L.W, L.C_phys, half, s);
         case L_CONV_TC:
@@ -1697,7 +1759,9 @@ bool patch_layout(const b2_engine* e, const Launch& L, BindPatch* p) {
     const bool half = e->half();
     switch (L.kind) {
         case L_INPUT_CAST:
-            if (L.k == 2) p->n_params = 8;                                  // input_cast_s2d_kernel(src, dst, N, C, H, W, pad_l, pad_r)
+            if (L.src_dtype == B2_DT_UINT8 && L.k == 2) p->n_params = 8;    // input_cast_u8_s2d_kernel(src, dst, N, H, W, pad_l, pad_r, nrm)
+            else if (L.src_dtype == B2_DT_UINT8) p->n_params = 6;           // input_cast_u8_c8_kernel(src, dst, N, H, W, nrm)
+            else if (L.k == 2) p->n_params = 8;                             // input_cast_s2d_kernel(src, dst, N, C, H, W, pad_l, pad_r)
             else if (half && L.C_phys == 8 && L.C <= 8) p->n_params = 5;    // input_cast_c8_kernel(src, dst, N, C, HW)
             else p->n_params = 6;                                           // input_cast_kernel(src, dst, N, C, HW, C_phys)
             p->in_index = 0;

@@ -1424,6 +1424,97 @@ int launch_input_cast_s2d(const void* src, bool src_half, void* dst, int N, int 
     return B2_LAUNCH_RC;
 }
 
+// uint8 HWC images -> normalised fp32 -> fp16 (round to nearest).  (x - mean) * inv_std is one rounded subtract and one
+// rounded multiply, never contracted into an FMA, so the values equal builder.preprocess_u8 bit for bit and the engine
+// computes exactly what its fp32 binding computes on the preprocessed batch.
+__device__ __forceinline__ float u8_norm(unsigned char v, float mean, float inv_std) {
+    return __fmul_rn(__fsub_rn(static_cast<float>(v), mean), inv_std);
+}
+
+// One thread per packed output pixel (a PAIR of crop pixels): consecutive threads read consecutive 2*C-byte runs of the
+// same source row, so a warp reads one contiguous span (no alignment assumed: crop_left * C may be odd).
+__global__ void input_cast_u8_s2d_kernel(const unsigned char* __restrict__ src, uint4* __restrict__ dst, int N, int H, int W,
+                                         int pad_l, int pad_r, U8Norm nrm) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const int W2 = W >> 1;
+    const int Wp = W2 + pad_l + pad_r;
+    const long long total = static_cast<long long>(N) * H * Wp, step = static_cast<long long>(gridDim.x) * blockDim.x;
+    for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total; idx += step) {
+        const int wp = static_cast<int>(idx % Wp);
+        const long long t = idx / Wp;
+        const int h = static_cast<int>(t % H);
+        const int n = static_cast<int>(t / H);
+        const int w2 = wp - pad_l;
+        uint4 o = make_uint4(0u, 0u, 0u, 0u);
+        if (w2 >= 0 && w2 < W2) {
+            const unsigned char* s =
+                src + ((static_cast<size_t>(n) * nrm.src_h + nrm.top + h) * nrm.src_w + nrm.left + 2 * w2) * nrm.C;
+            float f[8];
+#pragma unroll
+            for (int c = 0; c < 4; ++c) {
+                f[c] = f[4 + c] = 0.f;
+                if (c < nrm.C) {
+                    f[c] = u8_norm(__ldg(s + nrm.perm[c]), nrm.mean[c], nrm.inv_std[c]);
+                    f[4 + c] = u8_norm(__ldg(s + nrm.C + nrm.perm[c]), nrm.mean[c], nrm.inv_std[c]);
+                }
+            }
+            __half2* o2 = reinterpret_cast<__half2*>(&o);
+#pragma unroll
+            for (int i = 0; i < 4; ++i) o2[i] = __floats2half2_rn(f[2 * i], f[2 * i + 1]);
+        }
+        dst[idx] = o;
+    }
+}
+
+// One thread per crop pixel, one 16-byte store of 8 fp16 channels; a warp reads 32 * C contiguous source bytes.
+__global__ void input_cast_u8_c8_kernel(const unsigned char* __restrict__ src, uint4* __restrict__ dst, int N, int H, int W,
+                                        U8Norm nrm) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const long long total = static_cast<long long>(N) * H * W, step = static_cast<long long>(gridDim.x) * blockDim.x;
+    for (long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; idx < total; idx += step) {
+        const int w = static_cast<int>(idx % W);
+        const long long t = idx / W;
+        const int h = static_cast<int>(t % H);
+        const int n = static_cast<int>(t / H);
+        const unsigned char* s = src + ((static_cast<size_t>(n) * nrm.src_h + nrm.top + h) * nrm.src_w + nrm.left + w) * nrm.C;
+        float f[8];
+#pragma unroll
+        for (int c = 0; c < 8; ++c) f[c] = 0.f;
+#pragma unroll
+        for (int c = 0; c < 4; ++c)
+            if (c < nrm.C) f[c] = u8_norm(__ldg(s + nrm.perm[c]), nrm.mean[c], nrm.inv_std[c]);
+        uint4 o;
+        __half2* o2 = reinterpret_cast<__half2*>(&o);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) o2[i] = __floats2half2_rn(f[2 * i], f[2 * i + 1]);
+        dst[idx] = o;
+    }
+}
+
+int launch_input_cast_u8_s2d(const void* src, void* dst, int N, int H, int W, int pad_l, int pad_r, const U8Norm& nrm,
+                             int max_blocks, cudaStream_t stream) {
+    const long long total = static_cast<long long>(N) * H * (W / 2 + pad_l + pad_r);
+    const int threads = 256;
+    unsigned blocks = static_cast<unsigned>((total + threads - 1) / threads);
+    if (max_blocks > 0 && blocks > static_cast<unsigned>(max_blocks)) blocks = static_cast<unsigned>(max_blocks);  // grid-stride
+    B2_LAUNCH_RC = launch_kernel(input_cast_u8_s2d_kernel, dim3(blocks), dim3(threads), 0, stream, false,
+                                 static_cast<const unsigned char*>(src), reinterpret_cast<uint4*>(dst), N, H, W, pad_l, pad_r, nrm);
+    return B2_LAUNCH_RC;
+}
+
+int launch_input_cast_u8_c8(const void* src, void* dst, int N, int H, int W, const U8Norm& nrm, int max_blocks,
+                            cudaStream_t stream) {
+    const long long total = static_cast<long long>(N) * H * W;
+    const int threads = 256;
+    unsigned blocks = static_cast<unsigned>((total + threads - 1) / threads);
+    if (max_blocks > 0 && blocks > static_cast<unsigned>(max_blocks)) blocks = static_cast<unsigned>(max_blocks);  // grid-stride
+    B2_LAUNCH_RC = launch_kernel(input_cast_u8_c8_kernel, dim3(blocks), dim3(threads), 0, stream, false,
+                                 static_cast<const unsigned char*>(src), reinterpret_cast<uint4*>(dst), N, H, W, nrm);
+    return B2_LAUNCH_RC;
+}
+
 template <typename T>
 __global__ void output_cast_kernel(const T* __restrict__ src, float* __restrict__ dst, int N, int C, int HW,
                                    int C_phys) {

@@ -183,6 +183,22 @@ int launch_input_cast(const void* src, bool src_half, void* dst, int N, int C, i
 // border pixels zero)
 int launch_input_cast_s2d(const void* src, bool src_half, void* dst, int N, int C, int H, int W, int pad_l, int pad_r,
                           int max_blocks, cudaStream_t stream);
+// uint8 HWC image binding: source geometry, crop and normalisation (plan_format.h InputNormRec).  Passed BY VALUE as a
+// kernel argument, so the cast reads nothing but the image bytes.
+struct U8Norm {
+    float mean[4];
+    float inv_std[4];
+    int C;             // source channels, 1..4
+    int src_h, src_w;  // source image
+    int top, left;     // crop origin; the crop size is the engine tensor's H x W
+    int perm[4];       // output channel c reads source channel perm[c]
+};
+// uint8 [N, src_h, src_w, C] -> fp16 [N, H, pad_l + W/2 + pad_r, 8], the layout of launch_input_cast_s2d
+int launch_input_cast_u8_s2d(const void* src, void* dst, int N, int H, int W, int pad_l, int pad_r, const U8Norm& nrm,
+                             int max_blocks, cudaStream_t stream);
+// uint8 [N, src_h, src_w, C] -> fp16 NHWC [N, H, W, 8] (zero-filled channels C..7)
+int launch_input_cast_u8_c8(const void* src, void* dst, int N, int H, int W, const U8Norm& nrm, int max_blocks,
+                            cudaStream_t stream);
 // NHWC activations -> fp32 NCHW binding
 int launch_output_cast(const void* src, float* dst, int N, int C, int H, int W, int C_phys,
                        bool half_storage, cudaStream_t stream);

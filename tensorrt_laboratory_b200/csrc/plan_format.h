@@ -68,8 +68,19 @@ struct OpRec {  // 176 bytes
     uint64_t w_off, w_bytes, b_off, b_bytes;  // payload-relative
     // rectangular / anisotropic convs (0 = square: kw=k, stride_w=stride, pad_w_*=pad_).  `k`, `stride`, `pad_`
     // then describe the H direction.  INPUT_CAST: k = horizontal space-to-depth factor (0/1 = none, 2 = pack pixel
-    // pairs into channels [dw*4 + c]).
+    // pairs into channels [dw*4 + c]).  INPUT_CAST of a B2_DT_UINT8 binding: b_off / b_bytes address its InputNormRec
+    // (b_bytes = 48); 0 / 0 for every other input binding.
     uint32_t kw, stride_w, pad_w_lo, pad_w_hi;
+};
+// Normalisation of a uint8 HWC image binding (C <= 4), per item:
+//     y[c][h][w] = (float(x[crop_top + h][crop_left + w][perm[c]]) - mean[c]) * inv_std[c]      (fp32: one sub, one mul)
+// (H, W) is the crop = the engine tensor's geometry.  Entries c >= C are 0.
+struct InputNormRec {  // 48 bytes
+    float mean[4];
+    float inv_std[4];
+    uint32_t crop_top, crop_left;
+    uint8_t perm[4];
+    uint8_t pad[4];
 };
 struct BindingRec {  // 128 bytes
     char name[64];
@@ -87,5 +98,6 @@ static_assert(sizeof(TacticRec) == 40, "TacticRec size");
 static_assert(sizeof(TensorRec) == 96, "TensorRec size");
 static_assert(sizeof(OpRec) == 176, "OpRec size");
 static_assert(sizeof(BindingRec) == 128, "BindingRec size");
+static_assert(sizeof(InputNormRec) == 48, "InputNormRec size");
 
 }  // namespace b2plan

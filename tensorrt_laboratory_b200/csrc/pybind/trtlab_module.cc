@@ -33,6 +33,7 @@ py::dtype numpy_dtype(int b2_dtype) {  // same order as the reference's DataType
         case B2_DT_HALF: return py::dtype("float16");
         case B2_DT_INT8: return py::dtype::of<std::int8_t>();
         case B2_DT_INT32: return py::dtype::of<std::int32_t>();
+        case B2_DT_UINT8: return py::dtype::of<std::uint8_t>();
     }
     throw std::runtime_error("unknown binding dtype");
 }
@@ -84,6 +85,9 @@ struct PyInferRunner : public InferRunner {
             if (!b.isInput) throw py::value_error(key + " is not an input binding");
             py::array arr = py::array::ensure(item.second, py::array::c_style | py::array::forcecast);
             if (!arr) throw py::type_error(key + ": expected a numpy array");
+            // a uint8 image binding takes the image bytes: casting normalised floats to uint8 would wrap them silently
+            if (b.dtype == B2_DT_UINT8 && !arr.dtype().is(py::dtype::of<std::uint8_t>()))
+                throw py::type_error(key + ": this binding takes uint8 images, got dtype " + py::str(arr.dtype()).cast<std::string>());
             arr = py::array::ensure(arr.attr("astype")(numpy_dtype(int(b.dtype)), py::arg("copy") = false), py::array::c_style);
             if (arr.ndim() < 1) throw py::value_error(key + ": expected a leading batch dimension");
             const long batch = long(arr.shape(0));

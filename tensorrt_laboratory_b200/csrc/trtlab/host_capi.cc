@@ -393,7 +393,7 @@ int trt_device_throughput(const void* blob, size_t nbytes, int contexts, int bat
         int32_t dims[8];
         int nd = 0;
         b2_engine_binding_dims(eng, i, dims, &nd);
-        size_t n = b2_engine_binding_dtype(eng, i) == B2_DT_HALF ? 2 : 4;
+        size_t n = dtype_size(b2_engine_binding_dtype(eng, i));
         for (int d = 0; d < nd; ++d) n *= size_t(dims[d]);
         bytes[i] = n * size_t(b2_engine_max_batch(eng));
         if (b2_engine_binding_is_input(eng, i)) in_id = i;

@@ -32,8 +32,8 @@ _PKG = "nvidia.inferenceserver"
 SERVICE = _PKG + ".GRPCService"
 
 # model_config.proto DataType
-TYPE_FP16, TYPE_FP32, TYPE_INT8, TYPE_INT32 = 10, 11, 6, 8
-_NP_OF = {TYPE_FP32: np.float32, TYPE_FP16: np.float16, TYPE_INT8: np.int8, TYPE_INT32: np.int32}
+TYPE_UINT8, TYPE_FP16, TYPE_FP32, TYPE_INT8, TYPE_INT32 = 2, 10, 11, 6, 8
+_NP_OF = {TYPE_FP32: np.float32, TYPE_FP16: np.float16, TYPE_INT8: np.int8, TYPE_INT32: np.int32, TYPE_UINT8: np.uint8}
 _TYPE_OF = {np.dtype(v): k for k, v in _NP_OF.items()}
 # request_status.proto RequestStatusCode
 SUCCESS, UNKNOWN, INTERNAL, NOT_FOUND, INVALID_ARG, UNAVAILABLE = 1, 2, 3, 4, 5, 6
@@ -375,6 +375,8 @@ class RemoteInferRunner:
         batch = None
         for k, v in inputs.items():
             shape, dt = self._inputs[k]
+            if dt == np.uint8 and np.asarray(v).dtype != np.uint8:
+                raise TypeError(f"input '{k}' takes uint8 images, got {np.asarray(v).dtype}")
             a = np.ascontiguousarray(v, dtype=dt)
             if a.shape[1:] != shape:
                 if a.shape == shape:  # a single item without its batch dimension, as the reference accepts

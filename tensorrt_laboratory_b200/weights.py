@@ -69,3 +69,10 @@ def synthetic_input(batch: int, chw=(3, 224, 224), seed: int = 1234, ring: int =
     rng = np.random.default_rng(seed)
     shape = (ring, batch) + tuple(chw) if ring > 1 else (batch,) + tuple(chw)
     return rng.standard_normal(shape, dtype=np.float32)
+
+
+def synthetic_image_u8(batch: int, src_hw=(224, 224), channels: int = 3, seed: int = 1234, ring: int = 1) -> np.ndarray:
+    """uint8 [batch, src_h, src_w, C] images, uniform over 0..255 (what a JPEG decoder hands a uint8 image binding)."""
+    rng = np.random.default_rng(seed)
+    shape = (ring, batch) + tuple(src_hw) + (channels,) if ring > 1 else (batch,) + tuple(src_hw) + (channels,)
+    return rng.integers(0, 256, size=shape, dtype=np.uint8)
